@@ -1,7 +1,8 @@
 """TEST INFRASTRUCTURE ONLY — CPU restatement of the reference's noise schedule and DDIM sampler arithmetic.
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference leg may import this.
 Pinned by analytic known-answer values (SURVEY §8c) and against the unmodified reference sampler
-(tests/test_oracle_cpu.py (test_*_matches_reference_golden, test_oracle_matches_live_reference_unet), tests/golden/).  Paths cited are relative to /root/reference.
+(tests/test_oracle_cpu.py (test_*_matches_reference_golden*), tests/golden/).  Paths cited are relative to the reference
+repository's root.
 """
 from __future__ import annotations
 

@@ -2,9 +2,8 @@
 
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference leg may import this.
 It is a functional walk over a reference-keyed state dict (no nn.Modules), pinned against the UNMODIFIED
-reference by tests/test_oracle_cpu.py (test_*_matches_reference_golden, test_oracle_matches_live_reference_unet) (run in the authoring container, where /root/reference
-exists) and by the committed fixtures under tests/golden/ (generated from the reference by
-tests/golden/make_golden.py).
+reference by tests/test_oracle_cpu.py (test_*_matches_reference_golden*) through the committed fixtures under
+tests/golden/ (generated from the reference by tests/golden/make_golden*.py).
 
 Each function cites the reference lines it restates (paths relative to /root/reference).
 """

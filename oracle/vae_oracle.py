@@ -1,7 +1,7 @@
 """TEST INFRASTRUCTURE ONLY — CPU fp32 restatement of the dual-reference video decoder (and the encoder that
 produces its hidden states).  Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl
-reference leg may import this.  Pinned against the unmodified reference by tests/test_oracle_cpu.py (test_*_matches_reference_golden, test_oracle_matches_live_reference_unet) and
-tests/golden/.  Paths cited are relative to /root/reference.
+reference leg may import this.  Pinned against the unmodified reference by tests/test_oracle_cpu.py
+(test_*_matches_reference_golden*) and tests/golden/.  Paths cited are relative to the reference repository's root.
 """
 from __future__ import annotations
 

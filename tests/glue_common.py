@@ -1,36 +1,44 @@
-"""Shared by tests/golden/make_golden_glue.py (drives the UNMODIFIED reference) and tests/glue_driver.py (drives this
-repository's alias tree): the reference's own glue function scripts/evaluation/funcs.py::batch_ddim_sampling (:14-93) is
-loaded from /root/reference BY FILE and run unchanged on the tiny configuration.
+"""Shared by tests/golden/make_golden_glue.py (drives the UNMODIFIED reference with its own glue function
+scripts/evaluation/funcs.py::batch_ddim_sampling, :14-93) and tests/glue_driver.py (drives this repository's alias
+tree with `batch_ddim_sampling` below, which makes the same calls) on the tiny configuration.
 
 Conditioning stages (CLIP text / image towers, Resampler) are outside the hot path: both sides install the same seeded
 test doubles for `get_learned_conditioning`, `embedder` and `image_proj_model`."""
-import importlib.util
-import sys
-import types
-from pathlib import Path
-
 import torch
 
-REF_FUNCS = Path("/root/reference/scripts/evaluation/funcs.py")
 SEED_RNG = 77
 STEPS = 4
 
 
-def stub_io_modules():
-    """decord / cv2 are video-I/O imports at the top of funcs.py (absent here, never called on this path)."""
-    for name in ("decord", "cv2"):
-        if name not in sys.modules:
-            m = types.ModuleType(name)
-            m.VideoReader = m.cpu = None
-            sys.modules[name] = m
-
-
-def load_reference_funcs():
-    stub_io_modules()
-    spec = importlib.util.spec_from_file_location("reference_eval_funcs", REF_FUNCS)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
+def batch_ddim_sampling(model, cond, noise_shape, n_samples=1, ddim_steps=50, ddim_eta=1.0, cfg_scale=1.0, hs=None,
+                        temporal_cfg_scale=None, **kwargs):
+    """What the reference's inference scripts do around the model (funcs.py:14-93), for the case they run: an
+    "empty_seq" unconditional branch with a zero image token, DDIMSampler.sample with the scripts' keyword set
+    (clean_cond, temporal_length, conditional_guidance_scale_temporal, timestep spacing and guidance rescale chosen by
+    the latent width), then two dual-reference decodes, the second without frames 1 and T-2, whose two middle frames
+    replace the first decode's.  Returns [B, n_samples, C, T, H, W]."""
+    from lvdm.models.samplers.ddim import DDIMSampler            # the alias, as the scripts import it
+    sampler = DDIMSampler(model)
+    B, T = noise_shape[0], noise_shape[2]
+    fs = cond.pop("fs")
+    spacing, rescale = ("uniform", 0.0) if noise_shape[-1] == 32 else ("uniform_trailing", 0.7)
+    assert cfg_scale != 1.0 and model.uncond_type == "empty_seq"
+    uc_img = model.image_proj_model(model.embedder(torch.zeros(B, 3, 224, 224).to(model.device)))
+    uc = dict(cond, c_crossattn=[torch.cat([model.get_learned_conditioning(B * [""]), uc_img], dim=1)])
+    variants = []
+    for _ in range(n_samples):
+        samples, _ = sampler.sample(S=ddim_steps, conditioning=cond, batch_size=B, shape=noise_shape[1:], verbose=False,
+                                    unconditional_guidance_scale=cfg_scale, unconditional_conditioning=uc, eta=ddim_eta,
+                                    temporal_length=T, conditional_guidance_scale_temporal=temporal_cfg_scale,
+                                    x_T=None, fs=fs, timestep_spacing=spacing, guidance_rescale=rescale,
+                                    **dict(kwargs, clean_cond=True))
+        video = model.decode_first_stage(samples, ref_context=hs)
+        keep = [i for i in range(T) if i not in (1, T - 2)]
+        middle = model.decode_first_stage(samples[:, :, keep], ref_context=hs)
+        Tv = video.shape[2]
+        video[:, :, Tv // 2 - 1:Tv // 2 + 1] = middle[:, :, Tv // 2 - 2:Tv // 2]
+        variants.append(video)
+    return torch.stack(variants, dim=1)
 
 
 class _Fn(torch.nn.Module):
@@ -67,7 +75,7 @@ def glue_inputs(T, h, w, ctx_dim):
     return dict(frames=frames, c_concat=cc, prompts=prompts, mask=mask, x0=x0, fs=torch.tensor([10]))
 
 
-def run_glue(funcs, model, T, h, w, ctx_dim):
+def run_glue(batch_ddim_sampling, model, T, h, w, ctx_dim):
     """Two prompts back to back (a stale conditioning cache would show in the second), then prompt 0 again with the
     mask / x0 blending kwargs (ddim.py:174-180).  Returns the three decoded clips."""
     gi = glue_inputs(T, h, w, ctx_dim)
@@ -79,7 +87,7 @@ def run_glue(funcs, model, T, h, w, ctx_dim):
         for k, extra in ((0, {}), (1, {}), (0, dict(mask=gi["mask"], x0=gi["x0"]))):
             cond = {"c_crossattn": [gi["prompts"][k].clone()], "c_concat": [gi["c_concat"]], "fs": gi["fs"]}
             torch.manual_seed(SEED_RNG)
-            v = funcs.batch_ddim_sampling(model, cond, [1, 4, T, h, w], n_samples=1, ddim_steps=STEPS, ddim_eta=1.0,
-                                          cfg_scale=7.5, hs=hs, **extra)
+            v = batch_ddim_sampling(model, cond, [1, 4, T, h, w], n_samples=1, ddim_steps=STEPS, ddim_eta=1.0,
+                                    cfg_scale=7.5, hs=hs, **extra)
             outs.append(v.float())
     return outs

@@ -1,6 +1,6 @@
-"""Runs the reference's scripts/evaluation/funcs.py::batch_ddim_sampling UNCHANGED against this repository's alias tree
-(`lvdm.*` -> tooncrafter_b200) on the tiny configuration and saves the decoded clips.  Executed in a fresh interpreter
-by tests/test_reference_glue.py: this repository first on sys.path, /root/reference behind it (so the glue's
+"""Runs glue_common.batch_ddim_sampling — the calls the reference's inference scripts make around the model — against
+this repository's alias tree (`lvdm.*` -> tooncrafter_b200) on the tiny configuration and saves the decoded clips.
+Executed in a fresh interpreter by tests/test_reference_glue.py with this repository first on sys.path (so the glue's
 `from lvdm.models.samplers.ddim import DDIMSampler` and the YAML targets resolve to the aliases).
 
     python tests/glue_driver.py OUT.npz [cpu|cuda]
@@ -16,7 +16,6 @@ import torch
 HERE = Path(__file__).resolve().parent
 ROOT = HERE.parent
 sys.path[:0] = [str(ROOT), str(HERE)]
-sys.path.append("/root/reference")
 
 
 def main():
@@ -30,13 +29,14 @@ def main():
     if dev == "cpu":
         import ops_emulator
         runtime.TEST_EXECUTOR = ops_emulator.executor
+        # the interpreted programs are many small host ops: they stop scaling long before the core count of a large
+        # host, where oversubscribed threads make them slower instead
+        torch.set_num_threads(min(torch.get_num_threads(), 16))
     model = instantiate_from_config(model_config()).eval()
     synthetic.fill_module_(model, seed=0)
     model.perframe_ae = True
     model.temporal_length = TINY_T
     model = model.to(dev)
-    funcs = glue_common.load_reference_funcs()
-    assert funcs.DDIMSampler is alias_ddim.DDIMSampler
 
     # glue_common builds CPU inputs / doubles: move what the glue hands to the model onto the model's device
     real_run = glue_common.glue_inputs
@@ -55,7 +55,7 @@ def main():
         m.embedder = glue_common._Fn(lambda img: emb(img).to(dev))
         m.image_proj_model = glue_common._Fn(lambda t: proj(t.cpu()).to(dev))
     glue_common.install_conditioning_doubles = doubles_on_device
-    outs = glue_common.run_glue(funcs, model, TINY_T, *TINY_LATENT_HW, TINY_CONTEXT_DIM)
+    outs = glue_common.run_glue(glue_common.batch_ddim_sampling, model, TINY_T, *TINY_LATENT_HW, TINY_CONTEXT_DIM)
     np.savez_compressed(out, **{f"clip{i}": o.float().cpu().numpy() for i, o in enumerate(outs)})
     print("glue ok", [tuple(o.shape) for o in outs])
 
