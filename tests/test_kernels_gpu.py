@@ -491,7 +491,8 @@ def test_attention_cross_text_plus_image(ops):
 @pytest.mark.parametrize("Bs,T,L,heads,n_txt,n_img", [(2, 16, 2560, 5, 77, 16), (1, 3, 333, 2, 77, 16), (2, 2, 128, 1, 64, 32),
                                                        (1, 4, 640, 10, 77, 0)])
 def test_attention_cross_resident_kv_shapes(ops, Bs, T, L, heads, n_txt, n_img):
-    """The short-K/V cross-attention kernel at the UNet level-0 shape, with ragged query tiles, and with one segment."""
+    """The short-K/V cross-attention kernel at the UNet level-0 shape and with ragged query tiles; with one segment
+    (n_img = 0) the dispatch runs tc_attn3_kernel instead."""
     C = heads * 64
     N = Bs * T
     q = _rand(N, L, C, seed=171).half()
